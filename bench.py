@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
     python bench.py --impl reference ...                     CPU restatement of the reference path (oracle/)
+    python bench.py ... --dump-outputs DIR                   also write the last timed step's results as DIR/*.npy
 
 A step = one synthetic ScanNet-shaped scene (BASELINE.json configs[1]: ~200k voxels) through
   coordinate hashing + stride sets + kernel maps  ->  MinkUNet34C forward (768-d head)  ->
@@ -40,7 +41,38 @@ def parse():
     ap.add_argument('--match', default=None, choices=['cosine', 'ensemble'], help="matching step: cosine (default) or run/evaluate.py's ensemble path (default for config4_matterport)")
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--modules', action='store_true', help='time the module-by-module MinkowskiEngine surface instead of the fused engine')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last timed step returned as DIR/<name>.npy (see dump_outputs)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
+
+
+DUMP_ROWS = 8192          # rows of the wide per-voxel outputs kept by --dump-outputs (all rows of one scene: ~600 MB)
+
+
+def voxel_outputs(features, scores, labels):
+    """The per-voxel results of one step: every label, and features / scores at a fixed seeded sample of rows (rows.npy).
+    The inputs are seeded too, so two builds run with the same arguments can be compared file by file."""
+    rows = np.sort(np.random.RandomState(0).choice(len(labels), min(len(labels), DUMP_ROWS), replace=False))
+    idx = torch.from_numpy(rows).to(features.device)
+    return {'labels': labels.cpu().numpy(), 'rows': rows, 'features': features[idx].float().cpu().numpy(),
+            'scores': scores[idx].float().cpu().numpy()}
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: each array as <path>/<name>.npy, floating point as float32 (float64 stays float64), integers as
+    float64 (exact); 64 MB at most in all."""
+    conv = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        conv[name] = a.astype(np.float32 if a.dtype.kind == 'f' and a.dtype.itemsize <= 4 else np.float64)
+    total = sum(a.nbytes for a in conv.values())
+    assert total <= 64 << 20, f'--dump-outputs would write {total} bytes'
+    os.makedirs(path, exist_ok=True)
+    for name, a in conv.items():
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def peaks():
@@ -123,8 +155,9 @@ def crop_sample(coords, target):
     return coords[coords[:, 1] < cut]
 
 
-def cpu_pass(coords, arch, k_text, threads):
-    """One pass of the CPU restatement (oracle/) over `coords`: map building + forward + cosine matching."""
+def cpu_pass(coords, arch, k_text, threads, keep=False):
+    """One pass of the CPU restatement (oracle/) over `coords`: map building + forward + cosine matching.
+    keep: leave (features, scores, labels) in cpu_pass.last."""
     from openscene_b200 import synth
     from oracle import matching as om
     from oracle import me_cpu
@@ -139,8 +172,11 @@ def cpu_pass(coords, arch, k_text, threads):
     with torch.no_grad():
         out = model(me_cpu.SparseTensor(feats, torch.from_numpy(coords)))
         s = om._hmm(om._l2n(out), text)
-        s.max(1)
-    return time.perf_counter() - t0
+        label = s.max(1)[1]
+    dt = time.perf_counter() - t0
+    if keep:
+        cpu_pass.last = (out, s, label)
+    return dt
 
 
 cpu_pass.cache = {}
@@ -197,7 +233,9 @@ def run_reference(args, rank):
         coords = crop_sample(scene, max(4000, int(len(coords) * budget_s / (t_probe * total))))
     for _ in range(max(args.warmup - 1, 1 if coords is not scene else 0)):
         cpu_pass(coords, args.arch, args.k_text, threads)
-    ts = [cpu_pass(coords, args.arch, args.k_text, threads) for _ in range(args.steps)]
+    ts = [cpu_pass(coords, args.arch, args.k_text, threads, keep=i == args.steps - 1) for i in range(args.steps)]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, voxel_outputs(*cpu_pass.last))
     tot = sum(ts)
     value = len(coords) * args.steps / tot
     full = len(coords) == len(scene)
@@ -257,15 +295,19 @@ def run_distill(args, rank, local, world):
         loss_host.copy_(loss.reshape(1), non_blocking=True)
         return loss
 
+    last = {}
+
     def timed(fn, k):
         import gc
         gc.collect(); gc.disable()
         evs = []
-        for _ in range(k):
+        for i in range(k):
             flush.zero_()
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            a.record(); fn(); b.record()
+            a.record(); r = fn(); b.record()
             evs.append((a, b))
+            if i == k - 1:
+                last['loss'] = r
         torch.cuda.synchronize()
         gc.enable()
         seq = [a.elapsed_time(b) for a, b in evs]
@@ -290,6 +332,8 @@ def run_distill(args, rank, local, world):
     ms, stats = timed(step, args.steps)
     if sampler:
         sampler.sample(); sampler.nvml_reasons()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'loss': last['loss'].reshape(1).cpu().numpy()})
     launches = _cabi.lib().osb_launch_count() - l0
     barrier()
     ms_nosync = None
@@ -394,7 +438,7 @@ def main():
                 out = model(ME.SparseTensor(feats_dev, coords_dev))
         else:
             out = eng(coords_dev, feats_dev)
-        return match(out)
+        return out, match(out)
 
     label_host = [torch.empty(n0, dtype=torch.int64).pin_memory() for _ in range(4)]   # ring of pinned result buffers
     e2e_i = [0]
@@ -413,7 +457,7 @@ def main():
         buf.copy_(label, non_blocking=True)
         return buf
 
-    step_stats = {}
+    step_stats, last = {}, {}
 
     def timed(fn, k, sampler=None, tag=None):
         import gc
@@ -424,7 +468,10 @@ def main():
             for i in range(k):
                 flush.zero_()                                        # L2 flush, outside the timed events
                 a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                a.record(); fn(); b.record()
+                a.record(); r = fn(); b.record()
+                if tag and i == k - 1:
+                    last[tag] = r                            # only the last step's result outlives its step
+                del r
                 evs.append((a, b))
                 if sampler is not None and i in (k // 4, k // 2, (3 * k) // 4):
                     # on-device clock measurement, stream-ordered between two steps (outside their event pairs)
@@ -455,6 +502,10 @@ def main():
         sampler.nvml_reasons()                                 # ... and right after the timed region
     launches = _cabi.lib().osb_launch_count() - l0
     barrier()
+    if args.dump_outputs and rank == 0:
+        out, (scores, label, _) = last.pop('device')
+        dump_outputs(args.dump_outputs, voxel_outputs(out, scores, label))
+    last.clear()
     clocks = sampler.stop() if sampler else None
     for _ in range(2):
         step_e2e()

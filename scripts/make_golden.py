@@ -1,4 +1,4 @@
-"""Generate tests/golden/*.npz in the build container (needs /root/reference; NOT run on the GPU box).
+"""Generate tests/golden/*.npz from a checkout of the reference project (OpenScene), named by OSB_REFERENCE_ROOT.
 
 1. voxelizer_*.npz : outputs of the reference's own ``dataset/voxelizer.py`` (imported unmodified, with the
    ``collections.Sequence/Iterable`` aliases Python 3.12 needs) for seeded inputs + the exact 4x4 matrix it drew.
@@ -17,7 +17,16 @@
    synthetic scene / fused-feature files written to a scratch directory (``SharedArray`` stubbed; ``torch.load`` given
    the ``weights_only=False`` default of the PyTorch the reference targets), plus the 4x4 matrix its voxeliser drew.
 
-Usage: python scripts/make_golden.py [voxelizer] [unet] [fusion] [metric] [loader]
+6. ref_voxelizer_matrices.npz, ref_voxelizer_random.npz, ref_fusion_random.npz, ref_metric_random.npz : what the
+   reference's own ``Voxelizer``, ``PointCloudToImageMapper`` and metric functions return on the seeded random cases of
+   tests/test_voxelizer_matrix_vs_reference.py and tests/test_oracles_vs_reference_live.py.
+7. ref_models.npz  : the reference's ``models/mink_unet.py`` / ``models/disnet.py`` built on this repository's
+   ``MinkowskiEngine`` package: state-dict keys, shapes and a fixed sample of the seeded weights of every architecture
+   its factory accepts, plus the names it rejects (tests/test_reference_models_on_product.py).
+
+Usage: OSB_REFERENCE_ROOT=<reference checkout> python scripts/make_golden.py [voxelizer] [unet] [fusion] [metric] [loader]
+                                                                           [ref_random] [ref_models]
+(``ref_models`` imports this repository's MinkowskiEngine, ``unet`` the oracle's: run them in separate processes.)
 """
 import collections
 import collections.abc
@@ -28,7 +37,7 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = '/root/reference'
+REF = os.environ.get('OSB_REFERENCE_ROOT', '')
 sys.path.insert(0, ROOT)
 OUT = os.path.join(ROOT, 'tests', 'golden')
 
@@ -223,8 +232,122 @@ def golden_loader():
         shutil.rmtree(tmp, ignore_errors=True)
 
 
+def golden_ref_random():
+    """The reference's Voxelizer, PointCloudToImageMapper and metric functions on the random cases of the tests."""
+    from tests import test_oracles_vs_reference_live as to
+    from tests import test_voxelizer_matrix_vs_reference as tv
+    collections.Sequence = collections.abc.Sequence
+    collections.Iterable = collections.abc.Iterable
+    _stub_modules('tensorflow', 'tensorflow.io', 'tensorflow.compat', 'tensorflow.compat.v1',
+                  'open3d', 'clip', 'matplotlib', 'matplotlib.patches', 'matplotlib.pyplot')
+    sys.path.insert(0, REF)
+    sys.path.insert(0, os.path.join(REF, 'scripts', 'feature_fusion'))
+    from dataset.voxelizer import Voxelizer
+    from fusion_util import PointCloudToImageMapper
+    from util import metric as ref_metric
+    from util import util as ref_util
+
+    shape = (len(tv.FORMS), len(tv.MATRIX_SEEDS))
+    m_v, m_r, tail = np.zeros(shape + (4, 4)), np.zeros(shape + (4, 4)), np.zeros(shape + (4,))
+    for form in range(len(tv.FORMS)):
+        vox = Voxelizer(**tv.form_kwargs(form))
+        for seed in tv.MATRIX_SEEDS:
+            np.random.seed(seed)
+            m_v[form, seed], m_r[form, seed] = vox.get_transformation_matrix()
+            tail[form, seed] = np.random.rand(4)
+    np.savez_compressed(os.path.join(OUT, 'ref_voxelizer_matrices.npz'), m_v=m_v, m_r=m_r, tail=tail)
+
+    out = {}
+    for trial, pts, aug, vsize in tv.random_clouds():
+        n = len(pts)
+        vox = Voxelizer(voxel_size=vsize, clip_bound=None, use_augmentation=aug, scale_augmentation_bound=(0.9, 1.1),
+                        rotation_augmentation_bound=tv.ROT, translation_augmentation_ratio_bound=((-0.2, 0.2), (-0.2, 0.2), (0, 0)))
+        np.random.seed(trial)
+        M_v, M_r = vox.get_transformation_matrix()
+        np.random.seed(trial)                                     # same draws inside voxelize()
+        coords_aug, _, _, inds_rec, inds = vox.voxelize(pts, np.zeros((n, 3), np.float32), np.zeros(n, np.int64), return_ind=True)
+        out.update({f'matrix_{trial}': (M_r @ M_v) if aug else M_v, f'coords_{trial}': coords_aug,
+                    f'inds_{trial}': np.asarray(inds), f'inds_reverse_{trial}': np.asarray(inds_rec)})
+    np.savez_compressed(os.path.join(OUT, 'ref_voxelizer_random.npz'), **out)
+
+    out = {}
+    for seed, pts, poses, depths, intr, cut, thres in to.fusion_cases():
+        mapper = PointCloudToImageMapper(image_dim=(320, 240), intrinsics=intr, visibility_threshold=thres, cut_bound=cut)
+        maps = np.stack([mapper.compute_mapping(p, pts, d) for p, d in zip(poses, depths)])
+        assert maps.min() >= 0 and maps.max() < 1 << 15
+        out[f'mapping_{seed}'] = maps.astype(np.int16)
+    np.savez_compressed(os.path.join(OUT, 'ref_fusion_random.npz'), **out)
+
+    out = {}
+    orig_cuda = torch.Tensor.cuda
+    torch.Tensor.cuda = lambda self, *a, **k: self           # intersectionAndUnionGPU calls .cuda()
+    try:
+        for seed, C, ds, pred, gt, nofeat in to.metric_cases():
+            out[f'confusion_{seed}'] = ref_metric.confusion_matrix(pred.copy(), gt.copy(), C).astype(np.int64)
+            out[f'miou_{seed}'] = np.float64(ref_metric.evaluate(pred.copy(), gt.copy(), stdout=False, dataset=ds))
+            if not nofeat:
+                i_np, u_np, t_np = ref_util.intersectionAndUnion(pred.copy(), gt.copy(), C, 255)
+                i_t, u_t, t_t = ref_util.intersectionAndUnionGPU(torch.from_numpy(pred.copy()), torch.from_numpy(gt.copy()), C, 255)
+                for name, a, b in (('inter', i_np, i_t), ('union', u_np, u_t), ('target', t_np, t_t)):
+                    assert np.array_equal(a.astype(np.int64), b.numpy().astype(np.int64))
+                    out[f'{name}_{seed}'] = a.astype(np.int64)
+    finally:
+        torch.Tensor.cuda = orig_cuda
+    np.savez_compressed(os.path.join(OUT, 'ref_metric_random.npz'), **out)
+    print('ref_random written')
+
+
+def golden_ref_models():
+    """The reference's model files on this repository's MinkowskiEngine package: keys, shapes, sampled seeded weights."""
+    import importlib
+    import types
+    from tests import test_reference_models_on_product as tm
+    for name in [m for m in sys.modules if m.split('.')[0] in ('MinkowskiEngine', 'models')]:
+        del sys.modules[name]
+    import MinkowskiEngine as ME
+    assert ME.MinkowskiConvolution.__module__.startswith('openscene_b200')
+    sys.path.insert(0, REF)
+    mu = importlib.import_module('models.mink_unet')
+    dn = importlib.import_module('models.disnet')
+    assert os.path.realpath(mu.__file__).startswith(os.path.realpath(REF))
+    out = {}
+
+    def record(tag, model):
+        sd = model.state_dict()
+        out[f'{tag}_keys'] = np.array(list(sd.keys()))
+        out[f'{tag}_shapes'] = np.array([str(tuple(v.shape)) for v in sd.values()])
+        out[f'{tag}_sample'], out[f'{tag}_sums'] = tm.weight_sample(sd)
+
+    for arch in ('MinkUNet18A', 'MinkUNet34C'):
+        torch.manual_seed(0)
+        record(arch, mu.mink_unet(in_channels=3, out_channels=768, D=3, arch=arch))
+    for arch in tm.OTHER_ARCHS:
+        torch.manual_seed(0)
+        record(f'{arch}_20', mu.mink_unet(in_channels=3, out_channels=20, D=3, arch=arch))
+    for ext in ('openseg', 'lseg'):
+        torch.manual_seed(0)
+        record(f'DisNet_{ext}', dn.DisNet(cfg=types.SimpleNamespace(arch_3d='MinkUNet18A', feature_2d_extractor=ext)))
+    for arch in tm.REJECTED:
+        try:
+            mu.mink_unet(arch=arch)
+        except Exception:
+            continue
+        raise AssertionError(f'the reference accepts {arch}')
+    try:
+        mu.MinkUNet50(3, 20, 3)
+        raise AssertionError('the reference constructs MinkUNet50')
+    except TypeError:                                         # PLANES is None: self.PLANES[0] fails in network_initialization
+        pass
+    out['rejected'] = np.array(tm.REJECTED)
+    np.savez_compressed(os.path.join(OUT, 'ref_models.npz'), **out)
+    print('ref_models written')
+
+
 if __name__ == '__main__':
+    if not os.path.isdir(REF):
+        sys.exit('set OSB_REFERENCE_ROOT to a checkout of the reference project')
     os.makedirs(OUT, exist_ok=True)
-    todo = sys.argv[1:] or ['voxelizer', 'unet', 'fusion', 'metric', 'loader']
+    todo = sys.argv[1:] or ['voxelizer', 'unet', 'fusion', 'metric', 'loader', 'ref_random']
     for nm in todo:
-        {'voxelizer': golden_voxelizer, 'unet': golden_unet, 'fusion': golden_fusion, 'metric': golden_metric, 'loader': golden_loader}[nm]()
+        {'voxelizer': golden_voxelizer, 'unet': golden_unet, 'fusion': golden_fusion, 'metric': golden_metric, 'loader': golden_loader,
+         'ref_random': golden_ref_random, 'ref_models': golden_ref_models}[nm]()

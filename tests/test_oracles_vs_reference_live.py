@@ -1,95 +1,26 @@
-"""The CPU oracles against the REFERENCE's own functions, live, on random cases beyond the committed fixtures (build container
-only: needs /root/reference; the fixtures under tests/golden/ carry the same comparison to machines without the tree).
+"""The CPU oracles against what the REFERENCE's own functions returned on random cases beyond the other fixtures
+(tests/golden/ref_fusion_random.npz and ref_metric_random.npz, written by scripts/make_golden.py from the reference tree).
 
 * oracle/fusion_ref.compute_mapping  vs  scripts/feature_fusion/fusion_util.py: PointCloudToImageMapper.compute_mapping
 * oracle/metric_ref                  vs  util/metric.py (confusion_matrix, evaluate) and util/util.py (intersectionAndUnion[GPU])
 Bit-exact (integer work); mIoU to 1e-12."""
-import os
-import sys
-import types
-
 import numpy as np
 import pytest
-import torch
 
-REF = os.environ.get('OSB_REFERENCE_ROOT', '/root/reference')
-needs_ref = pytest.mark.skipif(not os.path.exists(os.path.join(REF, 'util', 'metric.py')),
-                               reason='reference tree not present on this machine')
+from tests.util import golden
 
 
-def _stub(*names):
-    made = []
-    for nm in names:
-        parts = nm.split('.')
-        for i in range(1, len(parts) + 1):
-            sub = '.'.join(parts[:i])
-            if sub not in sys.modules:
-                sys.modules[sub] = types.ModuleType(sub)
-                made.append(sub)
-            if i > 1:
-                setattr(sys.modules['.'.join(parts[:i - 1])], parts[i - 1], sys.modules[sub])
-    return made
-
-
-@pytest.fixture
-def ref_fusion_util():
-    made = _stub('tensorflow', 'tensorflow.io', 'tensorflow.compat', 'tensorflow.compat.v1')     # imported, never used by the mapper
-    path = os.path.join(REF, 'scripts', 'feature_fusion')
-    sys.path.insert(0, path)
-    sys.modules.pop('fusion_util', None)
-    try:
-        import fusion_util
-        yield fusion_util
-    finally:
-        sys.path.remove(path)
-        sys.modules.pop('fusion_util', None)
-        for m in made:
-            sys.modules.pop(m, None)
-
-
-@pytest.fixture
-def ref_metrics():
-    made = _stub('open3d', 'clip', 'matplotlib', 'matplotlib.patches', 'matplotlib.pyplot')
-    for name in [m for m in sys.modules if m == 'util' or m.startswith('util.') or m == 'dataset' or m.startswith('dataset.')]:
-        del sys.modules[name]
-    sys.path.insert(0, REF)
-    orig_cuda = torch.Tensor.cuda
-    torch.Tensor.cuda = lambda self, *a, **k: self           # intersectionAndUnionGPU calls .cuda(); no device here
-    try:
-        from util import metric as m, util as u
-        yield m, u
-    finally:
-        torch.Tensor.cuda = orig_cuda
-        sys.path.remove(REF)
-        for name in [m_ for m_ in sys.modules if m_ == 'util' or m_.startswith('util.') or m_ == 'dataset' or m_.startswith('dataset.')]:
-            del sys.modules[name]
-        for m_ in made:
-            sys.modules.pop(m_, None)
-
-
-@needs_ref
-def test_fusion_mapping_oracle_equals_the_reference_on_random_views(ref_fusion_util):
-    from oracle import fusion_ref
+def fusion_cases():
+    """(seed, points, poses, depths, intrinsics, cut bound, visibility threshold) of the eight view sets."""
     from openscene_b200.synth import fusion_case
-    n_vis = 0
     for seed in range(100, 108):
         with_depth = seed % 3 != 0
-        cut = [0, 5, 10, 20][seed % 4]
-        thres = [0.25, 0.1, 0.5][seed % 3]
         pts, poses, depths, intr = fusion_case(seed, 2500 + 300 * (seed % 5), with_depth)
-        mapper = ref_fusion_util.PointCloudToImageMapper(image_dim=(320, 240), intrinsics=intr, visibility_threshold=thres, cut_bound=cut)
-        for pose, depth in zip(poses, depths):
-            want = mapper.compute_mapping(pose, pts, depth)
-            got = fusion_ref.compute_mapping(pose, pts, depth, intr, (320, 240), cut, thres)
-            assert np.array_equal(got, want), seed
-            n_vis += int(want[:, 2].sum())
-    assert n_vis > 5000                                       # the cases exercise the visible branch
+        yield seed, pts, poses, depths, intr, [0, 5, 10, 20][seed % 4], [0.25, 0.1, 0.5][seed % 3]
 
 
-@needs_ref
-def test_metric_oracles_equal_the_reference_on_random_labels(ref_metrics):
-    from oracle import metric_ref
-    ref_metric, ref_util = ref_metrics
+def metric_cases():
+    """(seed, class count, dataset name, pred, gt, with 'no feature' predictions) of the six label sets."""
     for seed, (C, ds) in enumerate([(20, 'scannet_3d'), (21, 'matterport_3d'), (40, 'matterport_3d_40'), (80, 'matterport_3d_80'),
                                     (160, 'matterport_3d_160'), (16, 'nuscenes_3d')]):
         rng = np.random.RandomState(500 + seed)
@@ -101,13 +32,31 @@ def test_metric_oracles_equal_the_reference_on_random_labels(ref_metrics):
         nofeat = seed % 2 == 1
         if nofeat:
             pred[rng.rand(n) < 0.07] = 256
-        conf = ref_metric.confusion_matrix(pred.copy(), gt.copy(), C)
-        assert np.array_equal(metric_ref.confusion_matrix(pred, gt, C).astype(np.int64), conf.astype(np.int64)), ds
-        miou = ref_metric.evaluate(pred.copy(), gt.copy(), stdout=False, dataset=ds)
-        assert metric_ref.mean_iou(pred, gt, C)[0] == pytest.approx(float(miou), rel=1e-12), ds
+        yield seed, C, ds, pred, gt, nofeat
+
+
+def test_fusion_mapping_oracle_equals_the_reference_on_random_views():
+    from oracle import fusion_ref
+    g = golden('ref_fusion_random.npz')
+    n_vis = 0
+    for seed, pts, poses, depths, intr, cut, thres in fusion_cases():
+        want_all = g[f'mapping_{seed}']
+        assert len(want_all) == len(poses), seed
+        for pose, depth, want in zip(poses, depths, want_all):
+            got = fusion_ref.compute_mapping(pose, pts, depth, intr, (320, 240), cut, thres)
+            assert np.array_equal(got, want), seed
+            n_vis += int(want[:, 2].sum())
+    assert n_vis > 5000                                       # the cases exercise the visible branch
+
+
+def test_metric_oracles_equal_the_reference_on_random_labels():
+    from oracle import metric_ref
+    g = golden('ref_metric_random.npz')
+    for seed, C, ds, pred, gt, nofeat in metric_cases():
+        assert np.array_equal(metric_ref.confusion_matrix(pred, gt, C).astype(np.int64), g[f'confusion_{seed}']), ds
+        assert metric_ref.mean_iou(pred, gt, C)[0] == pytest.approx(float(g[f'miou_{seed}']), rel=1e-12), ds
         if not nofeat:
-            i_np, u_np, t_np = ref_util.intersectionAndUnion(pred.copy(), gt.copy(), C, 255)
-            i_t, u_t, t_t = ref_util.intersectionAndUnionGPU(torch.from_numpy(pred.copy()), torch.from_numpy(gt.copy()), C, 255)
+            # the reference's NumPy and torch versions agreed with each other when the fixture was made
             i, u, t = metric_ref.intersection_and_union(pred, gt, C)
-            for a, b, c in ((i, i_np, i_t), (u, u_np, u_t), (t, t_np, t_t)):
-                assert np.array_equal(a, b.astype(np.int64)) and np.array_equal(a, c.numpy().astype(np.int64)), ds
+            for a, name in ((i, 'inter'), (u, 'union'), (t, 'target')):
+                assert np.array_equal(a, g[f'{name}_{seed}']), (ds, name)

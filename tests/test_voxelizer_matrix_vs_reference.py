@@ -1,21 +1,15 @@
-"""Host half of the drop-in voxeliser against the REFERENCE's own class, live (build container only: needs /root/reference).
+"""Host half of the drop-in voxeliser against what the REFERENCE's own class returned (tests/golden/ref_voxelizer_*.npz,
+written by scripts/make_golden.py from the reference's ``dataset/voxelizer.py``).
 
 ``openscene_b200.voxelize.Voxelizer.get_transformation_matrix`` must consume the global NumPy RNG exactly as
 ``dataset/voxelizer.py:46-76`` does -- the loaders seed / share that stream (dataset/point_loader.py:58-61), so a different draw
-order would change every augmentation after it.  Compared bit for bit, matrices and RNG state, over the constructor forms the
-reference's loaders use; the NumPy oracle (oracle/voxelize_ref.py) is held to the same reference on random clouds beyond the four
-committed fixtures."""
-import collections
-import collections.abc
-import os
-import sys
-
+order would change every augmentation after it.  Compared bit for bit, matrices and the next draws of the stream, over the
+constructor forms the reference's loaders use; the NumPy oracle (oracle/voxelize_ref.py) is held to the same reference on random
+clouds beyond the four committed fixtures."""
 import numpy as np
 import pytest
 
-REF = os.environ.get('OSB_REFERENCE_ROOT', '/root/reference')
-needs_ref = pytest.mark.skipif(not os.path.exists(os.path.join(REF, 'dataset', 'voxelizer.py')),
-                               reason='reference tree not present on this machine')
+from tests.util import golden
 
 ROT = ((-np.pi / 64, np.pi / 64), (-np.pi / 64, np.pi / 64), (-np.pi, np.pi))        # point_loader.py:58-61
 FORMS = [
@@ -27,60 +21,44 @@ FORMS = [
     dict(voxel_size=0.02, use_augmentation=True, scale_augmentation_bound=(0.9, 1.1),
          rotation_augmentation_bound=(None, (-0.1, 0.1), (-np.pi, np.pi))),
 ]
+MATRIX_SEEDS = range(25)
 
 
-def _reference_voxelizer():
-    collections.Sequence = collections.abc.Sequence      # dataset/voxelization_utils.py:6 (Python 3.12)
-    collections.Iterable = collections.abc.Iterable      # dataset/voxelizer.py:55
-    for name in [m for m in sys.modules if m == 'dataset' or m.startswith('dataset.')]:
-        del sys.modules[name]
-    sys.path.insert(0, REF)
-    try:
-        from dataset.voxelizer import Voxelizer
-    finally:
-        sys.path.remove(REF)
-    return Voxelizer
+def form_kwargs(form):
+    return dict(FORMS[form], clip_bound=None, translation_augmentation_ratio_bound=((-0.2, 0.2), (-0.2, 0.2), (0, 0)),
+                ignore_label=255)
 
 
-@needs_ref
-@pytest.mark.parametrize('form', range(len(FORMS)))
-def test_matrix_and_rng_stream_equal_the_reference(form):
-    from openscene_b200.voxelize import Voxelizer as Mine
-    Ref = _reference_voxelizer()
-    kw = dict(FORMS[form], clip_bound=None, translation_augmentation_ratio_bound=((-0.2, 0.2), (-0.2, 0.2), (0, 0)), ignore_label=255)
-    ref, mine = Ref(**kw), Mine(**kw)
-    for seed in range(25):
-        np.random.seed(seed)
-        a_v, a_r = ref.get_transformation_matrix()
-        tail_ref = np.random.rand(4)                     # what the next consumer of the stream would see
-        np.random.seed(seed)
-        b_v, b_r = mine.get_transformation_matrix()
-        tail_mine = np.random.rand(4)
-        assert np.array_equal(a_v, b_v) and np.array_equal(a_r, b_r), (form, seed)
-        assert np.array_equal(tail_ref, tail_mine), "the two classes consumed the RNG stream differently"
-
-
-@needs_ref
-def test_oracle_equals_the_reference_on_random_clouds():
-    """oracle/voxelize_ref.py vs the reference's voxelize() beyond the committed fixtures: dense clouds with many duplicates,
-    negative coordinates, fp32 and fp64 inputs, augmentation on and off."""
-    from oracle import voxelize_ref
-    Ref = _reference_voxelizer()
+def random_clouds():
+    """(trial, points, augmentation on, voxel size): dense clouds with many duplicates, negative coordinates, fp32 and fp64."""
     rng = np.random.RandomState(2024)
     for trial in range(12):
         n = int(rng.randint(500, 6000))
         extent, shift = float(rng.uniform(0.3, 5.0)), float(rng.uniform(-3.0, 1.0))
         dtype = np.float32 if trial % 3 == 0 else np.float64
         pts = (rng.rand(n, 3) * extent + shift).astype(dtype)
-        aug = trial % 2 == 0
-        vox = Ref(voxel_size=float(rng.choice([0.02, 0.05, 0.1])), clip_bound=None, use_augmentation=aug,
-                  scale_augmentation_bound=(0.9, 1.1), rotation_augmentation_bound=ROT,
-                  translation_augmentation_ratio_bound=((-0.2, 0.2), (-0.2, 0.2), (0, 0)))
-        np.random.seed(trial)
-        M_v, M_r = vox.get_transformation_matrix()
-        rigid = (M_r @ M_v) if aug else M_v
-        np.random.seed(trial)
-        coords_aug, _, _, inds_rec, inds = vox.voxelize(pts, np.zeros((n, 3), np.float32), np.zeros(n, np.int64), return_ind=True)
-        cv, o_inds, o_inv, _ = voxelize_ref.voxelize(pts, rigid)
-        assert np.array_equal(cv, coords_aug), trial
-        assert np.array_equal(o_inds, np.asarray(inds)) and np.array_equal(o_inv, np.asarray(inds_rec)), trial
+        yield trial, pts, trial % 2 == 0, float(rng.choice([0.02, 0.05, 0.1]))
+
+
+@pytest.mark.parametrize('form', range(len(FORMS)))
+def test_matrix_and_rng_stream_equal_the_reference(form):
+    from openscene_b200.voxelize import Voxelizer as Mine
+    g = golden('ref_voxelizer_matrices.npz')
+    mine = Mine(**form_kwargs(form))
+    for seed in MATRIX_SEEDS:
+        np.random.seed(seed)
+        b_v, b_r = mine.get_transformation_matrix()
+        tail_mine = np.random.rand(4)                    # what the next consumer of the stream would see
+        assert np.array_equal(g['m_v'][form, seed], b_v) and np.array_equal(g['m_r'][form, seed], b_r), (form, seed)
+        assert np.array_equal(g['tail'][form, seed], tail_mine), "the two classes consumed the RNG stream differently"
+
+
+def test_oracle_equals_the_reference_on_random_clouds():
+    """oracle/voxelize_ref.py vs the reference's voxelize() beyond the committed fixtures, augmentation on and off; the
+    rigid matrix is the one the reference drew for the cloud."""
+    from oracle import voxelize_ref
+    g = golden('ref_voxelizer_random.npz')
+    for trial, pts, _, _ in random_clouds():
+        cv, o_inds, o_inv, _ = voxelize_ref.voxelize(pts, g[f'matrix_{trial}'])
+        assert np.array_equal(cv, g[f'coords_{trial}']), trial
+        assert np.array_equal(o_inds, g[f'inds_{trial}']) and np.array_equal(o_inv, g[f'inds_reverse_{trial}']), trial
