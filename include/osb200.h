@@ -246,6 +246,26 @@ int osb_match_ensemble(const float *feat3d, const void *feat2d_f16, int64_t n_vo
                        const void *text_f16, int32_t k_text, void *scores_f16, int64_t *label, void *feat_out_f16,
                        void *stream);
 
+/* Test-time repeats (run/evaluate.py:385-425): the product of osb_match_scores (feat2_f16 == NULL) or of
+ * osb_match_ensemble (feat = feat3d fp32, feat2_f16 = feat2d, sel_a = smax3d, sel_b = smax2d, normalize = 0), folded into
+ * a running fp16 sum instead of being written out:
+ *   h = fp16(a . text[k,:])                      the score osb_match_* returns
+ *   store[p,k] = first ? h + (+0.0) : h + store[p,k]   one fp16 rounding (== torch's `pred + store` on fp16 tensors;
+ *                                                     the first repeat turns -0 into +0 like `pred + 0.0`)
+ *   label[p]   = first argmax_k of the ACCUMULATED store[p,:] (== `store.float().max(1)[1]`; may be NULL)
+ *   store      in/out fp16 [n_pts, K]; read only when first == 0
+ * Limits as the tensor-core matcher: C in {512, 768}, 1 <= K <= 480.  Without inds_reverse n_pts must equal n_vox.
+ * There is no CUDA-core variant: under OSB_MATCH_SIMT=1 the call fails. */
+int osb_match_accumulate(const void *feat, int32_t feat_is_f16, const void *feat2_f16, const float *sel_a, const float *sel_b,
+                         int64_t n_vox, int32_t c, const int64_t *inds_reverse, int64_t n_pts, const void *text_f16,
+                         int32_t k_text, int32_t normalize, void *store_f16, int32_t first, int64_t *label, void *stream);
+/* Test-time repeats of class logits (run/eval_mink.py:168-216), CUDA cores, any C >= 1:
+ *   x = logits[inds_reverse[p], :] (fp32 [n_vox, C]; row p when inds_reverse is NULL, then n_pts == n_vox)
+ *   store[p,:] = first ? x + 0.0 : x + store[p,:]      (fp32 in/out [n_pts, C])
+ *   label_cur[p] = first argmax of x (this repeat alone), label_acc[p] = first argmax of store[p,:]; either may be NULL */
+int osb_logits_accumulate(const float *logits, int64_t n_vox, int32_t c, const int64_t *inds_reverse, int64_t n_pts,
+                          float *store, int32_t first, int64_t *label_cur, int64_t *label_acc, void *stream);
+
 /* Optional folded head (engine.forward_scores): rows z = [x L | x U] (fp32, row pitch ld floats) from one 1x1x1
  * convolution with the weights [L | U], W W^T = L L^T, U = W T^T  ->  score_k = fp16((x.U_k) / (|x L| + 1e-5)),
  * label = first argmax.  Same cosine scores as run/evaluate.py:305-310 without materialising the 768-d features. */

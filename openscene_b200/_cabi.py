@@ -51,6 +51,8 @@ SIGNATURES = {
     'osb_gather_rows_f32': (c_int, [P, P, I64, I32, P, P]),
     'osb_match_scores': (c_int, [P, I32, I64, I32, P, I64, P, I32, I32, P, P, P, P]),
     'osb_match_ensemble': (c_int, [P, P, I64, I32, P, I64, P, P, P, I32, P, P, P, P]),
+    'osb_match_accumulate': (c_int, [P, I32, P, P, P, I64, I32, P, I64, P, I32, I32, P, I32, P, P]),
+    'osb_logits_accumulate': (c_int, [P, I64, I32, P, I64, P, I32, P, P, P]),
     'osb_folded_head_finish': (c_int, [P, I64, I32, I32, I32, P, P, P, P]),
     'osb_voxelize_workspace_bytes': (SZ, [I64]),
     'osb_voxelize': (c_int, [P, I32, I64, POINTER(c_double), P, P, P, POINTER(I64), POINTER(c_double), P, SZ, P]),

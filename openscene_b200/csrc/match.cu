@@ -133,7 +133,8 @@ k_match_ensemble(const float *__restrict__ feat3d, const __half *__restrict__ fe
 // tensor-core implementation (match_tc.cu)
 int match_tc_run(const void *feat, int feat_is_f16, const void *feat2_f16, const float *sel_a, const float *sel_b, int c,
                  const int64_t *inds_reverse, int64_t n_pts, const void *text_f16, int k_text, int normalize,
-                 void *scores_f16, int64_t *label, float *smax, void *feat_out_f16, cudaStream_t stream);
+                 void *scores_f16, int64_t *label, float *smax, void *feat_out_f16, void *store_f16, int first,
+                 cudaStream_t stream);
 
 static bool use_simt() {   // OSB_MATCH_SIMT=1 selects the CUDA-core kernels below (cross-check path)
   static int v = -1;
@@ -160,7 +161,7 @@ int osb_match_scores(const void *feat, int32_t feat_is_f16, int64_t n_vox, int32
   if (n_pts == 0) return 0;
   if (!use_simt())
     return match_tc_run(feat, feat_is_f16, nullptr, nullptr, nullptr, c, inds_reverse, n_pts, text_f16, k_text, normalize,
-                        scores_f16, label, smax, nullptr, stream);
+                        scores_f16, label, smax, nullptr, nullptr, 0, stream);
   const unsigned grid = match_grid(n_pts);
   const __half2 *text = (const __half2 *)text_f16;
   __half *scores = (__half *)scores_f16;
@@ -187,7 +188,7 @@ int osb_match_ensemble(const float *feat3d, const void *feat2d_f16, int64_t n_vo
   if (n_pts == 0) return 0;
   if (!use_simt())
     return match_tc_run(feat3d, 0, feat2d_f16, smax3d, smax2d, c, inds_reverse, n_pts, text_f16, k_text, 0, scores_f16, label,
-                        nullptr, feat_out_f16, stream);
+                        nullptr, feat_out_f16, nullptr, 0, stream);
   const unsigned grid = match_grid(n_pts);
   if (c == 768)
     k_match_ensemble<12><<<grid, 256, 0, stream>>>(feat3d, (const __half *)feat2d_f16, inds_reverse, n_pts, smax3d, smax2d,
@@ -201,7 +202,85 @@ int osb_match_ensemble(const float *feat3d, const void *feat2d_f16, int64_t n_vo
   return 0;
 }
 
+int osb_match_accumulate(const void *feat, int32_t feat_is_f16, const void *feat2_f16, const float *sel_a, const float *sel_b,
+                         int64_t n_vox, int32_t c, const int64_t *inds_reverse, int64_t n_pts, const void *text_f16,
+                         int32_t k_text, int32_t normalize, void *store_f16, int32_t first, int64_t *label, void *stream_) {
+  OSB_CHECK(c == 512 || c == 768, "osb_match_accumulate: feature width %d unsupported (OpenScene uses 512 / 768)", c);
+  OSB_CHECK(k_text >= 1 && k_text <= 5 * 96, "osb_match_accumulate: K_text=%d outside 1..480 (one TMEM allocation)", k_text);
+  OSB_CHECK(n_vox > 0 && n_pts >= 0, "osb_match_accumulate: bad shape (n_vox=%lld, n_pts=%lld)", (long long)n_vox,
+            (long long)n_pts);
+  OSB_CHECK(inds_reverse != nullptr || n_pts == n_vox,
+            "osb_match_accumulate: without inds_reverse n_pts (%lld) must equal n_vox (%lld)", (long long)n_pts, (long long)n_vox);
+  OSB_CHECK(feat != nullptr && text_f16 != nullptr, "osb_match_accumulate: feat and text must not be NULL");
+  OSB_CHECK(store_f16 != nullptr, "osb_match_accumulate: store (fp16 [n_pts, K], read and written in place) is NULL");
+  OSB_CHECK(feat2_f16 == nullptr || (sel_a != nullptr && sel_b != nullptr),
+            "osb_match_accumulate: a second source needs both select arrays");
+  OSB_CHECK(!use_simt(), "osb_match_accumulate: no CUDA-core variant; OSB_MATCH_SIMT=1 cannot serve the accumulate epilogue");
+  if (n_pts == 0) return 0;
+  return match_tc_run(feat, feat_is_f16, feat2_f16, sel_a, sel_b, c, inds_reverse, n_pts, text_f16, k_text, normalize, nullptr,
+                      label, nullptr, nullptr, store_f16, first ? 1 : 0, (cudaStream_t)stream_);
+}
+
 }  // extern "C"
+
+// ---------------------------------------------------------------------------------------------------
+// Repeat accumulation of class logits (run/eval_mink.py:168-216): one warp per point gathers the voxel's fp32 logits row
+// through inds_reverse, folds it into the running fp32 sum (store = pred + 0.0 on the first repeat, pred + store after it)
+// and writes the first-maximum argmax of this repeat alone and of the accumulated row.  One pass instead of torch's
+// gather + add + two argmaxes over [N_pts, C].
+namespace osb {
+__device__ __forceinline__ void warp_argmax(float &best, int &best_k) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ob = __shfl_xor_sync(0xffffffffu, best, o);
+    const int ok = __shfl_xor_sync(0xffffffffu, best_k, o);
+    if (ob > best || (ob == best && ok < best_k)) { best = ob; best_k = ok; }
+  }
+}
+
+__global__ void __launch_bounds__(256)
+k_logits_accumulate(const float *__restrict__ logits, int c, const int64_t *__restrict__ inds_reverse, int64_t n_pts,
+                    float *__restrict__ store, int first, int64_t *__restrict__ label_cur, int64_t *__restrict__ label_acc) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t p = warp; p < n_pts; p += nwarps) {
+    const float *src = logits + (inds_reverse ? __ldg(inds_reverse + p) : p) * c;
+    float *st = store + p * c;
+    float bc = -INFINITY, ba = -INFINITY;
+    int kc = 0x7fffffff, ka = 0x7fffffff;
+    for (int k = lane; k < c; k += 32) {
+      const float v = __ldg(src + k);
+      const float s = __fadd_rn(v, first ? 0.f : st[k]);
+      st[k] = s;
+      if (k == lane || v > bc) { bc = v; kc = k; }       // a lane's first column seeds its candidate (rows of -inf)
+      if (k == lane || s > ba) { ba = s; ka = k; }
+    }
+    warp_argmax(bc, kc);
+    warp_argmax(ba, ka);
+    if (lane == 0) {
+      if (label_cur) label_cur[p] = kc;
+      if (label_acc) label_acc[p] = ka;
+    }
+  }
+}
+}  // namespace osb
+
+extern "C" int osb_logits_accumulate(const float *logits, int64_t n_vox, int32_t c, const int64_t *inds_reverse, int64_t n_pts,
+                                     float *store, int32_t first, int64_t *label_cur, int64_t *label_acc, void *stream_) {
+  OSB_CHECK(c >= 1 && n_vox > 0 && n_pts >= 0, "osb_logits_accumulate: bad shape (n_vox=%lld, C=%d, n_pts=%lld)",
+            (long long)n_vox, c, (long long)n_pts);
+  OSB_CHECK(inds_reverse != nullptr || n_pts == n_vox,
+            "osb_logits_accumulate: without inds_reverse n_pts (%lld) must equal n_vox (%lld)", (long long)n_pts, (long long)n_vox);
+  OSB_CHECK(logits != nullptr, "osb_logits_accumulate: logits is NULL");
+  OSB_CHECK(store != nullptr, "osb_logits_accumulate: store (fp32 [n_pts, C], read and written in place) is NULL");
+  if (n_pts == 0) return 0;
+  const unsigned grid = (unsigned)std::min<int64_t>(osb::ceil_div(n_pts, 8), 148 * 16);
+  osb::k_logits_accumulate<<<grid, 256, 0, (cudaStream_t)stream_>>>(logits, c, inds_reverse, n_pts, store, first ? 1 : 0,
+                                                                     label_cur, label_acc);
+  OSB_LAUNCH_CHECK();
+  return 0;
+}
 
 // ---------------------------------------------------------------------------------------------------
 // Folded head (optional fast path, openscene_b200/engine.py: forward_scores): the final 1x1x1 convolution

@@ -13,6 +13,11 @@
 // TMA (rows >= K_text are out of bounds -> zero fill), warp 17 issues `tcgen05.mma kind::f16` (M=128, N<=96 per pass,
 // K=16), warps 0-3 read the accumulators from TMEM, round to fp16, take the first-maximum argmax and write
 // scores / labels / row maxima.  HBM-bound: 4*C (or 2*C) bytes per point against 2*C*K flops.
+//
+// Accumulate epilogue (osb_match_accumulate, the test_repeats loop of run/evaluate.py:385-425): with `store` set, each
+// fp16 score h is folded into the caller's running fp16 sum instead of being written out -- store = h + 0.0 on the first
+// repeat (turns -0 into +0 like the reference's `pred + 0.0`), store = __hadd(h, store) after it (one fp16 rounding,
+// bit-identical to torch's fp32 add rounded to fp16) -- and the label is the first maximum of the ACCUMULATED row.
 #include "tc_ptx.cuh"
 #include <algorithm>
 
@@ -36,6 +41,8 @@ struct MatchTcParams {
   int64_t *label;                    // [n_pts] or NULL
   float *smax;                       // [n_pts] or NULL
   __half *feat_out;                  // [n_pts, C] or NULL: the fp16 operand actually multiplied (ensemble feature)
+  __half *store;                     // [n_pts, k_text] or NULL: running fp16 sum over repeats (accumulate epilogue)
+  int first;                         // store: 1 = first repeat (store is write-only)
 };
 
 __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t acc) {
@@ -207,7 +214,12 @@ k_match_tc(const __grid_constant__ CUtensorMap tmT, const MatchTcParams p) {
       for (int j = 0; j < 16; ++j) {
         const int k = col + j;
         if (k < p.k_text) {
-          const __half h = __float2half_rn(__uint_as_float(a[j]));
+          __half h = __float2half_rn(__uint_as_float(a[j]));
+          if (p.store != nullptr && pt < p.n_pts) {
+            __half *st = p.store + pt * p.k_text + k;
+            h = __hadd(h, p.first ? __float2half_rn(0.f) : *st);
+            *st = h;
+          }
           const float sc = __half2float(h);
           if (p.scores != nullptr && pt < p.n_pts) p.scores[pt * p.k_text + k] = h;
           if (sc > best) { best = sc; best_k = k; }
@@ -243,7 +255,8 @@ static int launch_match_tc(const MatchTcParams &p, const void *text_f16, cudaStr
 
 int match_tc_run(const void *feat, int feat_is_f16, const void *feat2_f16, const float *sel_a, const float *sel_b, int c,
                  const int64_t *inds_reverse, int64_t n_pts, const void *text_f16, int k_text, int normalize,
-                 void *scores_f16, int64_t *label, float *smax, void *feat_out_f16, cudaStream_t stream) {
+                 void *scores_f16, int64_t *label, float *smax, void *feat_out_f16, void *store_f16, int first,
+                 cudaStream_t stream) {
   MatchTcParams p{};
   p.feat = feat; p.feat2 = (const __half *)feat2_f16; p.sel_a = sel_a; p.sel_b = sel_b;
   p.inds_reverse = inds_reverse; p.n_pts = n_pts; p.C = c; p.k_text = k_text;
@@ -253,6 +266,7 @@ int match_tc_run(const void *feat, int feat_is_f16, const void *feat2_f16, const
   while (p.tmem_cols < p.n_pass * MT_NW) p.tmem_cols <<= 1;
   p.feat_is_f16 = feat_is_f16; p.normalize = normalize;
   p.scores = (__half *)scores_f16; p.label = label; p.smax = smax; p.feat_out = (__half *)feat_out_f16;
+  p.store = (__half *)store_f16; p.first = first;
   return launch_match_tc(p, text_f16, stream);
 }
 

@@ -65,3 +65,64 @@ def match_ensemble(predictions, feat_3d, inds_reverse, text_features, return_fea
         C.call('osb_match_ensemble', C.ptr(predictions), C.ptr(feat_3d), n_vox, c, C.ptr(inv), n_pts, C.ptr(smax3d),
                C.ptr(smax2d), C.ptr(text), k, C.ptr(scores), C.ptr(label), C.ptr(fe), C.stream_ptr())
     return scores, label, fe, smax3d < smax2d
+
+
+def _inds(inds_reverse, device, n_vox):
+    if inds_reverse is None:
+        return None, n_vox
+    inv = inds_reverse.to(device=device, dtype=torch.int64).contiguous()
+    return inv, inv.shape[0]
+
+
+def match_accumulate(feat, inds_reverse, text_features, store, first, normalize=False, feat2=None, smax3d=None, smax2d=None):
+    """One repeat of the ``test_repeats`` loop (run/evaluate.py:385-425) on the device: the fp16 scores of
+    ``_scores(feat, ...)`` -- or, with ``feat2`` (fp16 fused features) and the two row maxima, of the ensemble product --
+    are added into ``store`` (fp16 [N_pts, K], in place; ``first`` starts it from ``0.0 + pred``).  Returns the int64
+    labels ``store.float().max(1)[1]`` of the accumulated scores.  The [N_pts, K] scores are never materialised."""
+    C.require_cuda(feat, 'features')
+    feat = feat.contiguous()
+    is_f16 = feat.dtype == torch.float16
+    if not is_f16 and feat.dtype != torch.float32:
+        feat = feat.float()
+    n_vox, c = feat.shape
+    text = text_features.to(device=feat.device, dtype=torch.float16).contiguous()
+    k = text.shape[0]
+    if text.shape[1] != c:
+        raise ValueError(f"match_accumulate: text embeddings have width {text.shape[1]}, features {c}")
+    inv, n_pts = _inds(inds_reverse, feat.device, n_vox)
+    if store.dtype != torch.float16 or tuple(store.shape) != (n_pts, k) or not store.is_contiguous() or store.device != feat.device:
+        raise ValueError(f"match_accumulate: store must be a contiguous fp16 [{n_pts}, {k}] tensor on {feat.device}, "
+                         f"got {store.dtype} {tuple(store.shape)} on {store.device}")
+    if feat2 is not None:
+        if is_f16:
+            raise ValueError("match_accumulate: the ensemble product takes fp32 network features")
+        feat2 = feat2.to(feat.device, torch.float16).contiguous()
+        if feat2.shape != feat.shape:
+            raise ValueError(f"match_accumulate: fused features {tuple(feat2.shape)} vs network features {tuple(feat.shape)}")
+        smax3d, smax2d = smax3d.contiguous(), smax2d.contiguous()
+        if smax3d.shape != (n_pts,) or smax2d.shape != (n_pts,):
+            raise ValueError("match_accumulate: smax3d / smax2d must have one fp32 value per point")
+    with torch.cuda.device(feat.device):
+        label = torch.empty(n_pts, dtype=torch.int64, device=feat.device)
+        C.call('osb_match_accumulate', C.ptr(feat), int(is_f16), C.ptr(feat2), C.ptr(smax3d), C.ptr(smax2d), n_vox, c, C.ptr(inv),
+               n_pts, C.ptr(text), k, int(normalize), C.ptr(store), int(bool(first)), C.ptr(label), C.stream_ptr())
+    return label
+
+
+def logits_accumulate(logits, inds_reverse, store, first):
+    """One repeat of run/eval_mink.py:168-216 on the device: fp32 class logits [N_vox, C] gathered through
+    ``inds_reverse`` and added into ``store`` (fp32 [N_pts, C], in place; ``first`` starts it from ``pred + 0.0``).
+    Returns (label of this repeat alone, label of the accumulated store), both int64 first-maximum argmaxes."""
+    C.require_cuda(logits, 'logits')
+    logits = logits.float().contiguous()
+    n_vox, c = logits.shape
+    inv, n_pts = _inds(inds_reverse, logits.device, n_vox)
+    if store.dtype != torch.float32 or tuple(store.shape) != (n_pts, c) or not store.is_contiguous() or store.device != logits.device:
+        raise ValueError(f"logits_accumulate: store must be a contiguous fp32 [{n_pts}, {c}] tensor on {logits.device}, "
+                         f"got {store.dtype} {tuple(store.shape)} on {store.device}")
+    with torch.cuda.device(logits.device):
+        cur = torch.empty(n_pts, dtype=torch.int64, device=logits.device)
+        acc = torch.empty(n_pts, dtype=torch.int64, device=logits.device)
+        C.call('osb_logits_accumulate', C.ptr(logits), n_vox, c, C.ptr(inv), n_pts, C.ptr(store), int(bool(first)), C.ptr(cur),
+               C.ptr(acc), C.stream_ptr())
+    return cur, acc

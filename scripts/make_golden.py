@@ -24,8 +24,14 @@
    ``MinkowskiEngine`` package: state-dict keys, shapes and a fixed sample of the seeded weights of every architecture
    its factory accepts, plus the names it rejects (tests/test_reference_models_on_product.py).
 
+8. ref_repeats.npz : the reference's own ``run/evaluate.py:evaluate()`` and ``run/eval_mink.py:evaluate()`` with
+   ``test_repeats = 3``, run on the CPU over a fake loader / model that yield the seeded inputs of tests/repeats_ref.py
+   (``SparseTensor`` and ``Tensor.cuda`` patched to no-ops, ``precompute_text_related_properties`` to the seeded text and
+   mapper, ``metric.evaluate`` wrapped to record the labels it is given, the caller's concatenated per-repeat ``pred``
+   and the mIoU it returns).
+
 Usage: OSB_REFERENCE_ROOT=<reference checkout> python scripts/make_golden.py [voxelizer] [unet] [fusion] [metric] [loader]
-                                                                           [ref_random] [ref_models]
+                                                                           [ref_random] [ref_models] [ref_repeats]
 (``ref_models`` imports this repository's MinkowskiEngine, ``unet`` the oracle's: run them in separate processes.)
 """
 import collections
@@ -343,6 +349,93 @@ def golden_ref_models():
     print('ref_models written')
 
 
+def golden_ref_repeats():
+    """The reference's test_repeats loops on seeded inputs (tests/repeats_ref.py)."""
+    import importlib
+    import logging
+    import shutil
+    import tempfile
+    import types
+    from tests import repeats_ref as rr
+    collections.Sequence = collections.abc.Sequence
+    collections.Iterable = collections.abc.Iterable
+    _stub_modules('open3d', 'clip', 'matplotlib', 'matplotlib.patches', 'matplotlib.pyplot', 'tensorboardX', 'SharedArray')
+    sys.modules['tensorboardX'].SummaryWriter = object
+    sys.path.insert(0, REF)
+    ev = importlib.import_module('run.evaluate')
+    em = importlib.import_module('run.eval_mink')
+    from util import metric as ref_metric
+    assert os.path.realpath(ev.__file__).startswith(os.path.realpath(REF))
+    orig_cuda, orig_eval = torch.Tensor.cuda, ref_metric.evaluate
+    torch.Tensor.cuda = lambda self, *a, **k: self
+    calls = []
+
+    def recording_evaluate(pred_ids, gt_ids, stdout=False, dataset='scannet_3d'):
+        miou = orig_eval(pred_ids.copy(), gt_ids.copy(), stdout=False, dataset=dataset)
+        calls.append((np.asarray(pred_ids).copy(), sys._getframe(1).f_locals['pred'].clone(), miou, np.asarray(gt_ids).copy()))
+        return miou
+
+    ref_metric.evaluate = recording_evaluate
+    out = {}
+    tmp = tempfile.mkdtemp(prefix='osb_golden_')
+    try:
+        for name, (ftype, ds, k, c, n_scenes, R, nofeat, _) in sorted(rr.CASES.items()):
+            state = {}
+
+            class Loader:                                   # what the DataLoader yields: one scene per batch
+                dataset = types.SimpleNamespace(offset=0)      # evaluate.py sets it to the repeat; eval_mink.py does not
+                passes = 0
+
+                def __iter__(self):
+                    rep = self.passes
+                    self.passes += 1
+                    assert ftype == 'logits' or rep == self.dataset.offset
+                    for sc in range(n_scenes):
+                        state['key'] = (sc, rep)
+                        item = rr.scene_inputs(name, sc, rep)
+                        yield item if ftype != 'logits' else (item[0], item[1], item[2], item[5])
+
+                def __len__(self):
+                    return n_scenes
+
+            class Model(torch.nn.Module):                   # seeded voxel features for the scene / repeat being loaded
+                def forward(self, _sinput):
+                    sc, rep = state['key']
+                    return rr.voxel_features(name, sc, rep, len(rr.scene_inputs(name, sc, rep)[0]))
+
+            model = Model()
+
+            args = types.SimpleNamespace(test_repeats=R, feature_type=ftype, save_folder=tmp, model_path=tmp,
+                                         save_feature_as_numpy=False, mark_no_feature_to_unknown=nofeat, vis_input=False,
+                                         vis_pred=False, vis_gt=False, eval_iou=True, multiprocessing_distributed=False,
+                                         data_root=os.path.join(tmp, ds))
+            text, mapper = rr.text_and_mapper(name)
+            calls.clear()
+            if ftype == 'logits':
+                em.args, em.SparseTensor = args, (lambda f, c: None)
+                em.evaluate(model, Loader())
+                own, acc = calls[0::2], calls[1::2]
+                out[f'{name}_own_labels'] = np.stack([c_[0] for c_ in own])
+                out[f'{name}_own_miou'] = np.array([c_[2] for c_ in own])
+            else:
+                ev.args, ev.SparseTensor, ev.logger = args, (lambda f, c: None), logging.getLogger('osb_golden')
+                ev.precompute_text_related_properties = lambda _ls: (text, ['c%d' % i for i in range(k)], mapper, None)
+                ev.evaluate(model, Loader(), ds)
+                acc = calls
+            assert len(acc) == R
+            out[f'{name}_seed'] = np.int64(rr.case_seed(name))
+            out[f'{name}_gt'] = acc[0][3]
+            out[f'{name}_labels'] = np.stack([c_[0] for c_ in acc])
+            out[f'{name}_miou'] = np.array([c_[2] for c_ in acc])
+            out[f'{name}_pred'] = np.stack([c_[1].numpy() for c_ in acc])
+            print('ref_repeats', name, 'mIoU per prefix', out[f'{name}_miou'])
+    finally:
+        torch.Tensor.cuda, ref_metric.evaluate = orig_cuda, orig_eval
+        shutil.rmtree(tmp, ignore_errors=True)
+    np.savez_compressed(os.path.join(OUT, 'ref_repeats.npz'), **out)
+    print('ref_repeats written')
+
+
 if __name__ == '__main__':
     if not os.path.isdir(REF):
         sys.exit('set OSB_REFERENCE_ROOT to a checkout of the reference project')
@@ -350,4 +443,4 @@ if __name__ == '__main__':
     todo = sys.argv[1:] or ['voxelizer', 'unet', 'fusion', 'metric', 'loader', 'ref_random']
     for nm in todo:
         {'voxelizer': golden_voxelizer, 'unet': golden_unet, 'fusion': golden_fusion, 'metric': golden_metric, 'loader': golden_loader,
-         'ref_random': golden_ref_random, 'ref_models': golden_ref_models}[nm]()
+         'ref_random': golden_ref_random, 'ref_models': golden_ref_models, 'ref_repeats': golden_ref_repeats}[nm]()
